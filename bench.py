@@ -3,6 +3,9 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a kernels
     python bench.py --impl reference --steps K --warmup W    # reference arithmetic on the host cores (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + the last timed step's outputs as DIR/<name>.npy
+
+Every GPU measurement times K steps (calls); the `cpu_baseline` field is a fixed, bounded CPU sample (`--impl reference` times K of them).
 
 Workload (BASELINE.json configs[1]): `ssdnerf_cars_uncond`, batch 16 scenes per GPU, one STEP =
     50-step DDIM sample of a (3,6,128,128) triplane batch  ->  8-iteration occupancy-grid build  ->
@@ -44,6 +47,7 @@ METRIC = 'rays/sec (128^2 render) & DDIM triplanes/sec'
 UNET_FLOP_PER_SAMPLE_STEP = 217.96e9     # SURVEY.md §8d / Appendix B
 RAY_GATHER_BYTES_PER_SAMPLE = 288        # 3 planes x 4 taps x 6 ch x fp32 (SURVEY.md §8d)
 RAY_IO_BYTES = 20                        # image[3] + depth + weights_sum per ray
+DUMP_BYTES = 60_000_000                  # --dump-outputs writes at most this much array data (64 MB with the .npy headers)
 
 
 def orbit_poses(num, radius=2.6):
@@ -112,6 +116,22 @@ class ClockSampler:
                 if val.lower().startswith('active'):
                     reasons.add(name)
         return dict(sm_mhz=float(np.median(sm)) if sm else None, sm_max_mhz=mx, reasons=sorted(reasons), samples=len(sm))
+
+
+def dump_outputs(out_dir, arrays):
+    """`arrays` as DIR/<name>.npy in float32.  The budget of DUMP_BYTES is shared out smallest array first; an array larger than its
+    share is written as a sample of that many of its flattened elements, drawn with a fixed seed, so that two runs with the same
+    arguments write the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES // 4
+    for i, (name, t) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].numel())):
+        share = left // (len(arrays) - i)
+        a = t.detach()
+        if a.numel() > share:
+            idx = torch.randint(0, a.numel(), (share,), generator=torch.Generator().manual_seed(0)).sort().values
+            a = a.reshape(-1)[idx.to(a.device)]
+        left -= a.numel()
+        np.save(os.path.join(out_dir, name + '.npy'), a.float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------- this repo
@@ -196,7 +216,8 @@ def run_ours(args):
         return t0.elapsed_time(t1) / steps
 
     def resident_step(rec=None):
-        """one step with inputs already in HBM; stage boundaries marked with CUDA events on the launching stream"""
+        """one step with inputs already in HBM; stage boundaries marked with CUDA events on the launching stream -> what the step
+        hands its caller"""
         e = [ev() for _ in range(4)]
         e[0].record(stream)
         code = model.code_diff_pr_inv(diffusion(model.code_diff_pr(noise), return_loss=False)).contiguous()
@@ -207,7 +228,7 @@ def run_ours(args):
         e[3].record(stream)
         if rec is not None:
             rec.append(e)
-        return img
+        return dict(triplanes=code, density_grid=grid, density_bitfield=bitfield, image=img, depth=depth)
 
     # ---- end-to-end through the plugin API with host buffers (+ the eval-side NCCL all-gather of 8-bit images when N > 1)
     out_hosts = [torch.empty(B, V, 3, IMG, IMG, dtype=torch.float32).pin_memory() for _ in range(2)]
@@ -254,9 +275,9 @@ def run_ours(args):
             stream.wait_stream(side)
         stream.wait_stream(copy_stream)                 # every device->host copy has landed before the closing event
 
-    # ---- resident (kernel-side) measurement
+    # ---- resident (kernel-side) measurement; warm-up and timed steps alike keep the previous step's outputs alive until the next returns
     for _ in range(args.warmup):
-        resident_step()
+        last = resident_step()
     barrier()
     launches0 = L.ssdnerf_launch_count()
     clocks = ClockSampler(local); clocks.start()
@@ -264,10 +285,13 @@ def run_ours(args):
     t0, t1 = ev(), ev()
     t0.record(stream)
     for _ in range(args.steps):
-        resident_step(rec)
+        last = resident_step(rec)
     t1.record(stream)
     barrier()
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     total_ms = t0.elapsed_time(t1) / args.steps
     ddim_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in rec]))
     dens_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in rec]))
@@ -311,7 +335,7 @@ def run_ours(args):
         def render_s(counts=False):
             return R.render_fwd(R.DEC_S, planes_s, (128, 128), bits_s, dec_s.packed_blob(), poses=poses, intrinsics=intr, img_hw=(IMG, IMG),
                                 want_blend=True, want_counts=counts)
-        s_ms = timed(render_s, max(1, min(args.steps, 3)), 1)
+        s_ms = timed(render_s, args.steps, 1)
         s_samples = int(render_s(True)['num_samples'].sum().item())
         del code_s, planes_s
 
@@ -329,18 +353,18 @@ def run_ours(args):
         Sh.broadcast_scene(code1, bits1, 0)
         img, _ = model.render(decoder, code1, bits1, IMG, IMG, my_intr, my_poses, cfg=model.test_cfg)
         Sh.gather_views((img[0].clamp(0, 1) * 255.0 + 0.5).to(torch.uint8), V, out=ss_all, padded=ss_u8)
-    strong_ms = timed(strong_step, 10, 3)
+    strong_ms = timed(strong_step, args.steps, 3)
 
     # ---- stage-1 training step (every rank trains its own scenes; the shared decoder's gradient is all-reduced over NCCL inside the step)
     train = train2 = None
     if args.train:
-        train = train_measurement(dev, timed, rank)
-        train2 = train_stage2_measurement(dev, timed, rank)
+        train = train_measurement(dev, timed, rank, steps=args.steps)
+        train2 = train_stage2_measurement(dev, timed, rank, steps=args.steps)
 
     # ---- config-4 shape guided evaluations (rank 0): UNet forward + render loss forward/backward + UNet input-gradient pass
     guided = None
     if args.guided and rank == 0:
-        guided = guided_measurement(dev, ev, stream)
+        guided = guided_measurement(dev, ev, stream, args.steps)
 
     # ---- reduce over ranks (max time)
     times = torch.tensor([total_ms, ddim_ms, dens_ms, rend_ms, e2e_ms, s_ms or 0.0, strong_ms, train['ms'] if train else 0.0,
@@ -426,7 +450,7 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def train_measurement(dev, timed, rank, views=16, steps=4):
+def train_measurement(dev, timed, rank, steps, views=16):
     """`stage1_cars_recons16v` (reference config, resolved) at its own sizes: samples_per_gpu scenes x 16 views 128x128 per rank,
     `extra_scene_step` code-only Adam steps + ONE joint step of latents and decoder (weight gradients from the fused backward, gradient
     all-reduce over NCCL at N > 1) per train_step, 4096 rays per scene per step, scene cache write-back included."""
@@ -462,7 +486,7 @@ def train_measurement(dev, timed, rank, views=16, steps=4):
                                   f'{train_cfg["n_decoder_rays"]} rays/scene/step', 'last_log_vars': log})
 
 
-def train_stage2_measurement(dev, timed, rank, steps=4):
+def train_stage2_measurement(dev, timed, rank, steps):
     """`stage2_cars_uncond` (reference config, resolved): the denoiser (122 M parameters) trained on stored scene latents, samples_per_gpu
     scenes per rank: diffusion loss forward + UNet input / weight-gradient pass + Adam step; at N > 1 the gradient all-reduce (NCCL) is
     inside the step."""
@@ -493,9 +517,10 @@ def train_stage2_measurement(dev, timed, rank, steps=4):
                                   f'weight-gradient pass + Adam on 122 M parameters', 'last_log_vars': {k: v for k, v in log.items() if 'quartile' not in k}})
 
 
-def guided_measurement(dev, ev, stream, scenes=8, evals=6):
-    """BASELINE config 4 (`ssdnerf_chairs_recons1v`, reference config resolved): `evals` guided x_0 predictions at 8 scenes x one 128x128
-    conditioning view = what every DDIM / langevin step of val_guide costs (445 of them per batch in the shipped config)."""
+def guided_measurement(dev, ev, stream, steps, scenes=8, evals=6):
+    """BASELINE config 4 (`ssdnerf_chairs_recons1v`, reference config resolved): `steps` val_guide calls of `evals` guided x_0 predictions
+    each at 8 scenes x one 128x128 conditioning view = what every DDIM / langevin step of val_guide costs (445 of them per batch in the
+    shipped config)."""
     model, _ = build_model(dev, seed=1, rel='configs/paper_cfgs/ssdnerf_chairs_recons1v.py')
     diffusion, decoder = model.diffusion_ema, model.decoder_ema
     g = torch.Generator().manual_seed(5)
@@ -513,12 +538,13 @@ def guided_measurement(dev, ev, stream, scenes=8, evals=6):
     torch.cuda.synchronize(dev)
     a, b = ev(), ev()
     a.record(stream)
-    model.val_guide(data)
+    for _ in range(steps):
+        model.val_guide(data)
     b.record(stream)
     torch.cuda.synchronize(dev)
-    ms = a.elapsed_time(b) / evals
+    ms = a.elapsed_time(b) / (evals * steps)
     return {'workload': f'ssdnerf_chairs_recons1v (reference config): {scenes} scenes, 1 cond view {IMG}x{IMG}, grad_through_unet (default), '
-                        f'{evals} guided evaluations via val_guide', 'ms_per_guided_eval': ms, 'guided_evals_per_sec': 1e3 / ms,
+                        f'{steps} val_guide calls of {evals} guided evaluations', 'ms_per_guided_eval': ms, 'guided_evals_per_sec': 1e3 / ms,
             'rays_fwd_bwd_per_sec': scenes * IMG * IMG / (ms * 1e-3),
             'unet_fwd_bwd_tflops': 3 * UNET_FLOP_PER_SAMPLE_STEP * scenes / (ms * 1e-3) / 1e12,
             'note': 'flops = forward + data-gradient pass (2x forward) of the UNet only; includes the occupancy update and the fused render loss'}
@@ -609,7 +635,11 @@ def main():
     ap.add_argument('--no-side-s', dest='side_s', action='store_false', help='skip the variant-S renderer workload')
     ap.add_argument('--no-guided', dest='guided', action='store_false', help='skip the config-4 guided-evaluation measurement')
     ap.add_argument('--no-train', dest='train', action='store_false', help='skip the stage-1 training-step measurement')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the last timed step\'s triplanes, density grid / bitfield, images and '
+                    'depths as DIR/<name>.npy (float32; arrays beyond a 64 MB total are written as a seeded sample)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of --impl b200')
     if args.warmup < 3 and args.impl == 'b200':
         args.warmup = 3      # timing rule: at least 3 warm-up steps
     if args.impl == 'reference':

@@ -4,9 +4,10 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s ``cpu_baseline``
 ``--impl reference`` legs may import this package; ``ssdnerf_b200`` never does.
 
 PARITY UNPINNED BY REFERENCE TESTS: Lakonik/SSDNeRF ships no test-suite, golden
-vectors or CPU path for these kernels (SURVEY.md F2/F3).  The restatement is
-cross-checked on the GPU box against the reference's own CUDA kernels built into
-``oracle/_ref`` by ``oracle/build_ref.sh`` (``tests/test_ref_gpu.py``).
+vectors or CPU path for these kernels (SURVEY.md F2/F3).  The GPU kernels the
+tests hold to this restatement are in turn compared with the outputs of the
+reference's own CUDA kernels (built into ``oracle/_ref`` by ``oracle/build_ref.sh``),
+stored in ``tests/golden/reference_kernels_v1.npz`` (``tests/test_ref_gpu.py``).
 
 ``lib()`` returns the ctypes handle of ``oracle/_build/liboracle.so`` (compiled
 from ``ssdnerf_oracle.c`` with gcc on first use).

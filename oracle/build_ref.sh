@@ -1,8 +1,9 @@
 #!/usr/bin/env bash
 # Builds the REFERENCE's own CUDA kernels (lib/ops/raymarching, lib/ops/shencoder) from the sources where they lie under
 # /root/reference into oracle/_ref/ (git-ignored, travels to the GPU box), with ONE flag change: -std=c++14 -> -std=c++17
-# (PyTorch 2.11 headers need C++17; SURVEY.md F6).  Used by tests/test_ref_gpu.py as a GPU-side oracle and by
-# scripts/ref_gpu_baseline.py as the reference-GPU baseline.  No reference source is copied into the repo.
+# (PyTorch 2.11 headers need C++17; SURVEY.md F6).  Used by tests/golden/make_golden_ref_kernels.py to store the outputs
+# tests/test_ref_gpu.py compares against, and by tests/perf/ref_gpu_baseline.py as the reference-GPU baseline.
+# No reference source is copied into the repo.
 set -euo pipefail
 REF=${REF:-/root/reference}
 HERE="$(cd "$(dirname "$0")" && pwd)"

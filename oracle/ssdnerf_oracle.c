@@ -9,8 +9,10 @@
  * ships no tests, golden vectors or CPU path for these kernels (SURVEY.md F2/F3).
  * This restatement follows the arithmetic of the reference CUDA sources line by
  * line (citations below, file = lib/ops/raymarching/src/raymarching.cu unless
- * noted) and is cross-checked on the GPU box against the reference's own kernels
- * compiled into oracle/_ref/ (see oracle/build_ref.sh, tests/test_ref_gpu.py).
+ * noted).  The GPU kernels the tests hold to it are in turn compared with the
+ * outputs of the reference's own kernels (compiled into oracle/_ref/ by
+ * oracle/build_ref.sh), stored in tests/golden/reference_kernels_v1.npz
+ * (tests/test_ref_gpu.py).
  *
  * Arithmetic notes (SURVEY.md Appendix A):
  *  - nvcc contracts `o + t*d` into one FFMA; we use fmaf() at exactly those sites.

@@ -1,8 +1,7 @@
 """Resolves every python config the reference ships (configs/**/*.py, `_base_` inheritance followed by ssdnerf_b200.Config, the same
 semantics as mmcv.Config) and stores the parts the hot paths consume -- `model`, `train_cfg`, `test_cfg`, `data.samples_per_gpu` --
-as tests/golden/reference_configs.json.  Run in the build container (`python tests/golden/make_config_fixtures.py`); the GPU box has
-no /root/reference, so bench.py and the GPU tests build their models from this fixture: the reference's own settings, not a
-restatement.  tests/test_plugin_cpu.py re-derives the fixture from /root/reference when it exists and checks it is current."""
+as tests/golden/reference_configs.json.  Run as `REF=<checkout of the reference> python tests/golden/make_config_fixtures.py`;
+bench.py and the tests build their models from this fixture: the reference's own settings, not a restatement."""
 import glob
 import json
 import os
@@ -10,7 +9,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
-REF = '/root/reference'
+REF = os.environ.get('REF', '')
 
 
 def plain(x):
@@ -23,6 +22,8 @@ def plain(x):
 
 def resolve_all():
     from ssdnerf_b200 import Config
+    if not REF or not os.path.isdir(os.path.join(REF, 'configs')):
+        raise SystemExit(f'REF={REF!r} is not a checkout of the reference (set REF to one)')
     out = {}
     for path in sorted(glob.glob(os.path.join(REF, 'configs', '**', '*.py'), recursive=True)):
         cfg = Config.fromfile(path)

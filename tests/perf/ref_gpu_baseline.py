@@ -15,8 +15,8 @@ torch.backends.cudnn.benchmark = True
 
 
 def ref_render(params, code_single, bf, ro, rd, max_steps=256):
-    from tests.test_ref_gpu import _reference_eval_loop
-    return _reference_eval_loop(rmref, shref, params, ro, rd, code_single, bf, max_steps=max_steps)
+    from tests.golden.make_golden_ref_kernels import reference_eval_loop
+    return reference_eval_loop(rmref, shref, params, ro, rd, code_single, bf, max_steps=max_steps)
 
 
 def time_render(V):

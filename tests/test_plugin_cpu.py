@@ -9,7 +9,7 @@ import ssdnerf_b200 as S
 from oracle import unet_port as up
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
+REFERENCE_CONFIGS = os.path.join(ROOT, 'tests', 'golden', 'reference_configs.json')
 
 
 def test_registry_names():
@@ -35,11 +35,17 @@ def test_build_from_repo_config_and_state_dict_keys():
     assert m.code_diff_pr_inv(torch.zeros(2, 18, 128, 128)).shape == (2, 3, 6, 128, 128)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference checkout only exists in the build container')
 @pytest.mark.parametrize('cfg_rel', ['configs/paper_cfgs/ssdnerf_cars_uncond.py', 'configs/paper_cfgs/ssdnerf_chairs_recons1v.py',
                                      'configs/paper_cfgs/ssdnerf_abotables_uncond.py'])
-def test_reference_configs_build_unchanged(cfg_rel):
-    cfg = S.Config.fromfile(os.path.join(REF, cfg_rel))
+def test_reference_configs_build_unchanged(cfg_rel, tmp_path):
+    """the reference's config as resolved into tests/golden/reference_configs.json (tests/golden/make_config_fixtures.py), loaded back
+    through Config.fromfile from a `_base_` file and a file overriding its test_cfg, as the reference composes its configs"""
+    import json
+    ref = json.load(open(REFERENCE_CONFIGS))[cfg_rel]
+    (tmp_path / 'base.py').write_text(f"model = {ref['model']!r}\ntrain_cfg = {ref['train_cfg']!r}\ntest_cfg = dict(num_timesteps=-1)\n")
+    (tmp_path / 'cfg.py').write_text(f"_base_ = 'base.py'\ntest_cfg = {ref['test_cfg']!r}\n")
+    cfg = S.Config.fromfile(str(tmp_path / 'cfg.py'))
+    assert json.loads(json.dumps(cfg)) == {k: ref[k] for k in ('model', 'train_cfg', 'test_cfg')}
     m = S.build_model(cfg.model, train_cfg=cfg.get('train_cfg'), test_cfg=cfg.get('test_cfg'))
     assert type(m).__name__ == 'DiffusionNeRF'
     assert m.diffusion.test_cfg['num_timesteps'] == cfg.test_cfg['num_timesteps']
@@ -47,16 +53,13 @@ def test_reference_configs_build_unchanged(cfg_rel):
 
 def test_every_reference_config_builds_from_the_fixture():
     """tests/golden/reference_configs.json = every config the reference ships, resolved (tests/golden/make_config_fixtures.py); each one
-    builds through the registry unchanged, and the fixture is current with /root/reference when that exists"""
+    builds through the registry unchanged"""
     import json
-    cfgs = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'reference_configs.json')))
+    cfgs = json.load(open(REFERENCE_CONFIGS))
     assert len(cfgs) == 24
     for name, c in cfgs.items():
         m = S.build_model(c['model'], train_cfg=c['train_cfg'], test_cfg=c['test_cfg'])
         assert type(m).__name__ in ('DiffusionNeRF', 'MultiSceneNeRF'), name
-    if os.path.isdir(REF):
-        from tests.golden.make_config_fixtures import resolve_all
-        assert json.loads(json.dumps(resolve_all(), sort_keys=True)) == cfgs
     # the bench / GPU-test config is the fixture entry, and the repo's restated config file agrees with it
     own = S.Config.fromfile(os.path.join(ROOT, 'configs', 'cars_uncond_b200.py'))
     refc = cfgs['configs/paper_cfgs/ssdnerf_cars_uncond.py']
